@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — rows/s of the hot path on B200, next to the HBM roofline and the reference's CPU path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload zillow|q6|c1] [--rows R] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload zillow|q6|c1] [--rows R] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the stage over the whole synthetic workload. Default workload = BASELINE.json
 configs[1]: the Zillow Z1 pipeline over 100M synthetic rows (cyclic replication of the reference's 32,661-row
@@ -39,12 +39,108 @@ def parse_args():
     ap.add_argument("--cpu-sample-rows", type=int, default=1_000_000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--keys", type=int, default=0, help="distinct keys of the aggbykey workload (default rows/100)")
-    ap.add_argument("--min-region-s", type=float, default=2.0,
-                    help="the K-step timed region is repeated (each repeat bracketed by barrier + synchronize) until this much time has "
-                         "been measured; the reported time is the median repeat")
+    ap.add_argument("--min-region-s", type=float, default=0.0,
+                    help="repeat the K-step timed region (each repeat bracketed by barrier + synchronize) until this much time has "
+                         "been measured and report the median repeat; by default the K steps run once")
     ap.add_argument("--no-pageable", action="store_true", help="skip the pageable-host-memory end-to-end variant")
     ap.add_argument("--no-extras", action="store_true", help="default workload only: skip the brief c1 / aggregateByKey measurements")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the headline workloads' last timed step returned to DIR/*.npy "
+                         f"(float32 / float64, at most {DUMP_LIMIT >> 20} MB; rank 0; see OutputDump)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what this project's timed path computed: use it with --impl ours")
+    return args
+
+
+DUMP_LIMIT = 64 << 20  # bytes of .npy data one --dump-outputs run writes at most
+
+
+class OutputDump:
+    """--dump-outputs DIR: what a workload's timed path returned in its last timed step, as DIR/<workload>.<array>.npy in float32 or
+    float64, so that two builds of the project can be compared output for output (the inputs are generated from fixed seeds).
+
+      <wl>.result            aggregate stages: the aggregate of every block (one value per block)
+      <wl>.rows              row stages: number of output rows; the rows are the output of every block in block order (hash
+                             tables: the groups sorted by value, their order in the table is not part of the result)
+      <wl>.sample            indices of the rows written: all of them, or a fixed, seeded sample when they exceed the size limit
+      <wl>.<NN_col>          a fixed-width output column (float64; i64 values beyond 2^53 are rounded)
+      <wl>.<NN_col>.bytes    a string column: the bytes of the sampled rows (float32, one value per byte; absent when all are empty) ...
+      <wl>.<NN_col>.lengths  ... and their lengths
+      <wl>.<NN_col>.valid    an Option column: 1 = the row holds a value
+      <wl>.exceptions.*      the same for the exception records (row in block, row number, code, operator id)
+    No array of length 0 is written: a table without rows is only its .rows file."""
+
+    def __init__(self, path, n_workloads):
+        os.makedirs(path, exist_ok=True)
+        self.path = path
+        self.limit = (DUMP_LIMIT - (1 << 20)) // n_workloads  # 1 MB left for the .npy headers and the one-value arrays
+
+    def _save(self, name, a):
+        np.save(os.path.join(self.path, name + ".npy"), a)
+
+    def aggregate(self, wl_name, values):
+        self._save(f"{wl_name}.result", np.array(values, np.float64))
+
+    def rows(self, wl_name, prog, blocks, exceptions, sort=False):
+        """blocks: the output columns (backend.Column) of every block of stage `prog`; exceptions: the EXC_DTYPE records of every block."""
+        from tuplex_b200.backend import EXC_DTYPE, Column
+        from tuplex_b200.ir import T_I64
+        names = [(prog.out_names[i] if i < len(prog.out_names) else None) or f"col{i}" for i in range(len(blocks[0]))]
+        exc = np.concatenate(exceptions) if exceptions else np.zeros(0, EXC_DTYPE)
+        exc_cols = [Column(T_I64, np.ascontiguousarray(exc[f])) for f in EXC_DTYPE.names]
+        self._table(f"{wl_name}.exceptions", list(EXC_DTYPE.names), [[c] for c in exc_cols], self.limit // 8, False)
+        self._table(wl_name, names, [[b[c] for b in blocks] for c in range(len(names))], self.limit - self.limit // 8, sort)
+
+    def _table(self, prefix, names, parts, limit, sort):
+        from tuplex_b200.ir import T_STR
+        cols = []
+        for ps in parts:  # one column over the blocks: fixed-width values, or string bytes + row starts + lengths
+            present = None
+            if any(p.valid is not None for p in ps):
+                present = np.concatenate([p.present() if p.valid is not None else np.ones(len(p), bool) for p in ps])
+            if ps[0].type == T_STR:
+                base = np.cumsum([0] + [len(p.data) for p in ps])
+                starts = np.concatenate([p.offsets[:-1].astype(np.int64) + b for p, b in zip(ps, base)])
+                lens = np.concatenate([np.diff(p.offsets.astype(np.int64)) for p in ps])
+                cols.append((np.concatenate([p.data for p in ps]), starts, lens, present))
+            else:
+                cols.append((np.concatenate([p.data for p in ps]).astype(np.float64), None, None, present))
+        n = len(cols[0][0]) if cols[0][1] is None else len(cols[0][1])
+        order = np.arange(n)
+        if sort and n:
+            keys = []
+            for data, starts, lens, present in cols:
+                if starts is not None:
+                    data = np.unique(np.array([data[s:s + l].tobytes() for s, l in zip(starts, lens)], dtype=object).astype(bytes),
+                                     return_inverse=True)[1]
+                keys += [data] + ([present] if present is not None else [])
+            order = np.lexsort(keys[::-1])
+        row_bytes = np.full(n, 8, np.int64)  # its index in <prefix>.sample
+        for _, starts, lens, present in cols:
+            row_bytes += 8 if starts is None else 8 + 4 * lens
+            row_bytes += 0 if present is None else 4
+        idx = np.arange(n)
+        if row_bytes.sum() > limit:
+            cand = np.random.default_rng(0).choice(n, size=min(n, limit // 8), replace=False)
+            idx = np.sort(cand[np.cumsum(row_bytes[order[cand]]) <= limit])
+        rows = order[idx]
+        self._save(f"{prefix}.rows", np.array([n], np.float64))
+        if n == 0:  # no arrays of length 0: the row count says that there is nothing
+            return
+        self._save(f"{prefix}.sample", idx.astype(np.float64))
+        for i, (name, (data, starts, lens, present)) in enumerate(zip(names, cols)):
+            stem = "%s.%02d_%s" % (prefix, i, "".join(ch if ch.isalnum() else "_" for ch in name))
+            if starts is None:
+                self._save(stem, data[rows])
+            else:
+                ln = lens[rows]
+                pos = np.repeat(starts[rows] - (np.cumsum(ln) - ln), ln) + np.arange(int(ln.sum()))
+                if len(pos):
+                    self._save(stem + ".bytes", data[pos].astype(np.float32))
+                self._save(stem + ".lengths", ln.astype(np.float64))
+            if present is not None:
+                self._save(stem + ".valid", present[rows].astype(np.float32))
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -577,9 +673,9 @@ def measure_join(args, rank, world, local, dist):
     return out
 
 
-def measure(args, wl_key, rank, world, local, dist, hc):
-    """Device-resident `value`, `roofline`, end-to-end `e2e` (page-locked and pageable host inputs) and the CPU arm of one workload.
-    Returns the fields of its JSON object (rank 0) or None."""
+def measure(args, wl_key, rank, world, local, dist, hc, dump=None):
+    """Device-resident `value`, `roofline`, end-to-end `e2e` (page-locked and pageable host inputs) and the CPU arm of one workload;
+    with `dump` (an OutputDump), what the last timed step returned is written. Returns the fields of its JSON object (rank 0) or None."""
     import torch
     from tuplex_b200 import backend, ir
     wargs = argparse.Namespace(**vars(args))
@@ -613,11 +709,14 @@ def measure(args, wl_key, rank, world, local, dist, hc):
             tot = ir.bits_f64(st.agg_finish(local, [ir.f64_bits(tot)])[0])
         return tot
 
-    def step_resident():
+    kept = []  # with keep=True: the results a caller of the step receives, freed once they are dumped
+
+    def step_resident(keep=False):
         kms = 0.0
         launches = 0
         n_out = 0
         partials = []
+        keep_rows = keep and ep == ir.C["TPLX_EP_MEMORY"]
         if ep == ir.C["TPLX_EP_HASH"]:
             st.hash_reset(local)
             st.hash_reserve(local, wl.get("nkeys", 1 << 20))
@@ -627,20 +726,24 @@ def measure(args, wl_key, rank, world, local, dist, hc):
             inf = r.info
             out = (inf.kernel_ms, inf.kernel_launches, int(inf.n_out_rows),
                    ir.bits_f64(r.aggregate_bits()[0]) if ep == ir.C["TPLX_EP_AGGREGATE"] else None, int(inf.specialised_launches))
+            if keep_rows:
+                return out, r
             r.free()
-            return out
+            return out, None
         # row stages: blocks in flight on the GPU's execution lanes (the latency-bound dense launch of one block overlaps the
         # prefilter of the next). Aggregate scans are DRAM-bound (nothing to overlap) and hash stages share one table per
         # device: those run one block at a time.
         runner = pool.map if ep == ir.C["TPLX_EP_MEMORY"] else map
         spec = 0
-        for km, kl, no, part, sl in runner(one_resident, dev_blocks):
+        for (km, kl, no, part, sl), r in runner(one_resident, dev_blocks):
             kms += km
             launches += kl
             spec += sl
             n_out += no
             if part is not None:
                 partials.append(part)
+            if r is not None:
+                kept.append(r)
         if ep == ir.C["TPLX_EP_AGGREGATE"]:
             stats["result"] = combine_partials(partials)
         if ep == ir.C["TPLX_EP_HASH"]:
@@ -650,7 +753,10 @@ def measure(args, wl_key, rank, world, local, dist, hc):
             n_out = int(fin.info.n_out_rows)
             kms += fin.info.kernel_ms
             launches += fin.info.kernel_launches
-            fin.free()
+            if keep:
+                kept.append(fin)
+            else:
+                fin.free()
         stats.update(kernel_ms=kms, launches=launches, n_out=n_out, specialised=spec)
 
     def step_e2e(blocks):
@@ -715,23 +821,30 @@ def measure(args, wl_key, rank, world, local, dist, hc):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t[0])
 
-    W = max(args.warmup, 3)
-    for _ in range(W):
-        step_resident()
+    # the sampler starts before the warm-up, so that starting nvidia-smi does not compete with the timed steps for the host
     clocks = Clocks(local)
     clocks.start()
-    # the K-step region is repeated until min_region_s of it has been measured (a 20-step region of this stage is well under
-    # a second); every repeat is K steps between barrier + synchronize, the reported one is the median repeat (max over ranks)
+    W = max(args.warmup, 3)
+    for i in range(W):
+        # with --dump-outputs the last warm-up step holds its results like the dumped step will, so that the device memory pool
+        # already holds that much when the timed steps run
+        step_resident(keep=dump is not None and i == W - 1)
+    # K steps between barrier + synchronize; with --min-region-s the region is repeated until that much time has been measured
+    # and the median repeat is reported (max over ranks)
     reps = []
     kms = 0.0
     launches = 0
     spent = 0.0
     while True:
-        kacc = lacc = 0
+        kacc = lacc = done = 0
+        for r in kept:  # held by the last warm-up step or a previous repeat's last step
+            r.free()
+        kept.clear()
 
         def one_step():
-            nonlocal kacc, lacc
-            step_resident()
+            nonlocal kacc, lacc, done
+            done += 1
+            step_resident(keep=dump is not None and done == args.steps)
             kacc += stats["kernel_ms"]
             lacc += stats["launches"]
         dt_r = max_over_ranks(timed(one_step, args.steps))
@@ -741,6 +854,15 @@ def measure(args, wl_key, rank, world, local, dist, hc):
             break
     reps.sort()
     dt, kms, launches = reps[len(reps) // 2]
+    if dump is not None:
+        if ep == ir.C["TPLX_EP_AGGREGATE"]:
+            dump.aggregate(wl["name"], [stats["result"]])
+        else:
+            dump.rows(wl["name"], prog, [r.columns() for r in kept], [r.exceptions() for r in kept] if ep == ir.C["TPLX_EP_MEMORY"] else [],
+                      sort=ep == ir.C["TPLX_EP_HASH"])
+        for r in kept:
+            r.free()
+        kept.clear()
 
     # end-to-end through the C ABI with host buffers (H2D of inputs + D2H of results inside the timed region), K steps
     step_e2e(wl["blocks"])
@@ -758,7 +880,7 @@ def measure(args, wl_key, rank, world, local, dist, hc):
             del pb
         except MemoryError:
             dt_pg = None
-    clk = clocks.stop()  # sampled over all timed regions (device-resident repeats and end-to-end steps)
+    clk = clocks.stop()  # sampled over the warm-up and all timed regions (device-resident steps and end-to-end steps)
 
     line = None
     if rank == 0:
@@ -863,7 +985,8 @@ def main():
         tdist.init_comm(local)  # this rank's NCCL communicator inside libtplx_gpu.so (id broadcast over the launcher's group)
     hc = host_cores()
     keys = ["zillow", "q6"] if args.workload == "both" else [args.workload]
-    parts = {k: measure(args, k, rank, world, local, dist, hc) for k in keys}
+    dump = OutputDump(args.dump_outputs, len(keys)) if args.dump_outputs and rank == 0 else None
+    parts = {k: measure(args, k, rank, world, local, dist, hc, dump) for k in keys}
     extras = {}
     if args.workload == "both" and not args.no_extras:
         # the other two configurations of BASELINE.json, measured briefly in the same run (device-resident value + roofline + e2e):
@@ -979,7 +1102,9 @@ def main_csv(args, rank, world, local):
         if dist is not None:
             dist.barrier()
 
-    def run_block(buf, fetch):
+    kept = []  # with keep=True: (parse, result) of every buffer, freed once they are dumped
+
+    def run_block(buf, fetch, keep=False):
         p = buf.parse(types, delimiter=delim, header=has_header, lazy=lazy)
         r = st.run(p.block, 0)
         inf, pinf = r.info, p.info
@@ -992,13 +1117,16 @@ def main_csv(args, rank, world, local):
                 nb += c.nbytes()
         out = (float(pinf.parse_ms), float(inf.kernel_ms), int(pinf.kernel_launches) + int(inf.kernel_launches), int(inf.n_out_rows),
                int(pinf.n_rows), int(pinf.n_bad), sum(int(x) for x in p.block_bytes()), nb)
-        r.free()
-        p.free()
+        if keep:
+            kept.append((p, r))
+        else:
+            r.free()
+            p.free()
         return out
 
-    def step_resident():
+    def step_resident(keep=False):
         acc = [0.0, 0.0, 0, 0, 0, 0, 0, 0]
-        for o in map(lambda b: run_block(b, False), bufs):
+        for o in map(lambda b: run_block(b, False, keep), bufs):
             for i, v in enumerate(o):
                 acc[i] += v
         stats.update(parse_ms=acc[0], stage_ms=acc[1], launches=acc[2], n_out=acc[3], rows=acc[4], bad=acc[5], col_bytes=acc[6])
@@ -1014,24 +1142,40 @@ def main_csv(args, rank, world, local):
             d2h += o[7]
         stats["d2h"] = d2h
 
-    for _ in range(max(args.warmup, 3)):
-        step_resident()
+    dumping = args.dump_outputs is not None and rank == 0
+    n_warm = max(args.warmup, 3)
+    for i in range(n_warm):
+        step_resident(keep=dumping and i == n_warm - 1)  # the device memory pool grows to what the dumped step holds
     assert stats["rows"] == total and stats["bad"] == 0 and (expect_out is None or stats["n_out"] == expect_out), stats
     if expect_agg is not None:  # one buffer = `cycles` copies of the generated rows
         assert abs(stats["agg"] - cycles * expect_agg) <= 1e-9 * abs(cycles * expect_agg), (stats["agg"], cycles * expect_agg)
+    for p, r in kept:
+        r.free()
+        p.free()
+    kept.clear()
     clocks = Clocks(local)
     sync_all()
     clocks.start()
     t0 = time.perf_counter()
     pms = sms = 0.0
     launches = 0
-    for _ in range(args.steps):
-        step_resident()
+    for i in range(args.steps):
+        step_resident(keep=dumping and i == args.steps - 1)
         pms += stats["parse_ms"]
         sms += stats["stage_ms"]
         launches += stats["launches"]
     sync_all()
     dt = time.perf_counter() - t0
+    if kept:
+        dump = OutputDump(args.dump_outputs, 1)
+        if is_agg:
+            dump.aggregate(name, [ir.bits_f64(r.aggregate_bits()[0]) for _, r in kept])
+        else:
+            dump.rows(name, prog, [r.columns() for _, r in kept], [r.exceptions() for _, r in kept])
+        for p, r in kept:
+            r.free()
+            p.free()
+        kept.clear()
     e2e_steps = max(1, min(args.steps, 3))
     step_e2e()
     sync_all()

@@ -80,3 +80,29 @@ def zillow_reference_udfs():
 
 
 zillow_reference_udfs()
+
+
+def csvmonkey_cells():
+    """tests/golden/csvmonkey_cells.npz = what the reference's own csvmonkey reader (oracle/_ref/csv_ref) makes of
+    the cell-splitting vectors of tests/test_csv_oracle.py::test_cells_equal_reference_csvmonkey:
+      inputs / input_offsets   1,540 inputs with pathological quoting (seeded), concatenated
+      cells / cell_offsets     the reader's cell dump of each input
+      zillow_sha256            sha256 of its cell dump of tests/golden/zillow_noexc.csv.gz (the dump itself is 7.7 MB)"""
+    import random
+    sys.path[:0] = [ROOT, os.path.dirname(HERE)]
+    from oracle import pyoracle as po
+    from csv_helpers import T_BOOL, T_F64, T_I64, T_STR, gen_csv
+    rng = random.Random(7)
+    alpha = ["a", "b", '"', ",", "\n", "\r", " ", "1", "x", '""', ',"', '"\n', '",', "\r\n"]
+    inputs = ["".join(rng.choice(alpha) for _ in range(rng.randint(0, 60))).encode() for _ in range(1500)]
+    inputs += [gen_csv(rng, 30, [T_I64, T_STR, T_F64, T_STR, T_BOOL], dirty=0.2, weird_quotes=0.05) for _ in range(40)]
+    cells = [po.csv_ref_cells(s) for s in inputs]
+    offs = lambda parts: np.cumsum([0] + [len(p) for p in parts], dtype=np.uint64)
+    zillow = gzip.open(os.path.join(HERE, "zillow_noexc.csv.gz"), "rb").read()
+    np.savez_compressed(os.path.join(HERE, "csvmonkey_cells.npz"),
+                        inputs=np.frombuffer(b"".join(inputs), np.uint8), input_offsets=offs(inputs),
+                        cells=np.frombuffer(b"".join(cells), np.uint8), cell_offsets=offs(cells),
+                        zillow_sha256=np.frombuffer(hashlib.sha256(po.csv_ref_cells(zillow)).digest(), np.uint8))
+
+
+csvmonkey_cells()
